@@ -219,6 +219,30 @@ def read_peaks():
         return 6650.0, "fallback 6.65 TB/s (B200_PROFILING.md)"
 
 
+DUMP_SAMPLE_UNITS = 256        # units whose produced texts --dump-outputs writes (<= 256 x 20 KiB x 4 B: well under 64 MB)
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """--dump-outputs: each array as DIR/<name>.npy.  Integer fields go out as float64 (exact below 2**53), bytes as float32."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float32 if a.dtype == np.uint8 else np.float64))
+
+
+def sampled_texts(out, oo, n: int):
+    """The produced texts of a fixed, seeded sample of the units: (unit indices, their bytes concatenated, offsets into those bytes)."""
+    import numpy as np
+
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, DUMP_SAMPLE_UNITS), replace=False))
+    parts = [out[int(oo[i]):int(oo[i + 1])] for i in idx]
+    offs = np.zeros(len(parts) + 1, dtype=np.int64)
+    np.cumsum([len(x) for x in parts], out=offs[1:])
+    return idx, (np.concatenate(parts) if parts else np.zeros(0, dtype=np.uint8)), offs
+
+
 def chain_config(world: int, units: int):
     return {"workload": "configs[3] semantics at 16 KiB: full tool_post_invoke chain — harmful_content_detector (9 IGNORECASE regexes) + regex_filter (2 rules, rewrite "
                         f"on match) + toon_encoder (JSON->TOON, kept when smaller); valid JSON payloads, {int(MIX[0][1]*100)}% tabular / {int(MIX[1][1]*100)}% nested config / "
@@ -339,6 +363,8 @@ def main():
     ap.add_argument("--units", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--hit-rate", type=float, default=1e-4)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed (rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     chain = args.workload == "chain"
@@ -475,6 +501,11 @@ def main():
     toon_ms = [each[i] for i in range(1, kn.value, 2)]
     v_res = last["v"].copy()
     out_res, oo_res = engine.device_output(ctx), last["oo"].copy()       # un-timed copy of the resident outputs, for the parity checks below
+    if args.dump_outputs and rank == 0:
+        # the verdict record of every unit, and the texts produced (rewritten or TOON) for a fixed sample of the units
+        idx, sample, sample_offs = sampled_texts(out_res, oo_res, n)
+        dump_outputs(args.dump_outputs, {"verdict_match_bitmap": v_res["match_bitmap"], "verdict_flags": v_res["flags"], "verdict_out_len": v_res["out_len"],
+                                         "verdict_aux": v_res["aux"], "text_sample_units": idx, "text_sample_bytes": sample, "text_sample_offsets": sample_offs})
 
     for _ in range(2):
         step_cabi()
@@ -765,6 +796,9 @@ def scan_bench(args, rank, local_rank, world):
     launches = ctx.kernel_launches - l0
     clocks = sampler.stop() if sampler else None
     cand, steps_dfa = ctx.scan_counters()
+    if args.dump_outputs and rank == 0:
+        # the match bitmaps of every unit (W words of 64 pattern bits each) the last timed scan wrote
+        dump_outputs(args.dump_outputs, {"match_bitmap": d_bms[(step_no[0] - 1) & 1 if world > 1 else 0].cpu().numpy().view(np.uint64).reshape(n, W)})
     for _ in range(2):
         step_e2e()
     e2e_steps = max(3, min(args.steps, 10))

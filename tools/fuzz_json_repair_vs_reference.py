@@ -1,7 +1,7 @@
 """Container-only: live differential fuzz of the json_repair drop-in (on the engine's CPU simulator: JSON kernel source for "does it parse",
 substitution routines for the trailing-comma rule) against the REFERENCE'S OWN plugins/json_repair/json_repair.py, imported unmodified from
 /root/reference (orjson stood in for by the strict stdlib parser; texts that would expose an orjson / json delta are skipped).
-usage: python tools/fuzz_json_repair_vs_reference.py [seed] [cases]"""
+usage: python tools/fuzz_json_repair_vs_reference.py [--record OUT] [seed] [cases]  |  --replay tests/golden/fuzz_json_repair.json.gz"""
 import os
 import random
 import re
@@ -18,29 +18,11 @@ from fuzz_toon_tp import make_gen  # noqa: E402
 _DELTA = re.compile(r"\d{18,}|[eE][+-]?\d{3,}|\\u[dD][89a-fA-F]|NaN|Infinity")
 
 
-def main() -> int:
-    if not os.path.isdir(gen_golden.REF):
-        print("fuzz_json_repair_vs_reference: /root/reference is not here (container-only tool)")
-        return 0
-    seed = int(sys.argv[1]) if len(sys.argv) > 1 else 1
-    n = int(sys.argv[2]) if len(sys.argv) > 2 else 3000
-    gen_golden.install_shims()
-    import pytest
-    from cpex.framework import GlobalContext, PluginConfig, PluginContext, ToolPostInvokePayload
-    from plugins.json_repair.json_repair import JSONRepairPlugin as RefPlugin
-
-    import hostsim_batcher
-    import test_json_repair as tj
-    from mcp_context_forge_b200.plugins.json_repair import JSONRepairPlugin
-
-    hostsim_batcher.install(pytest.MonkeyPatch())
-    ref = RefPlugin(PluginConfig(name="jr", kind="x", hooks=["tool_post_invoke"]))
-    ctx = PluginContext(global_context=GlobalContext(request_id="fuzz"))
+def texts(seed: int, n: int):
     rng = random.Random(seed)
     case = make_gen(rng)
-    t0 = time.time()
-    cases = []
-    while len(cases) < n:
+    out = []
+    while len(out) < n:
         t = case()
         k = rng.random()
         if k < 0.25:
@@ -49,20 +31,67 @@ def main() -> int:
             t = re.sub(r"([}\]])", lambda m: rng.choice([",", ", ", ",\n", "", ""]) + m.group(1), t)
         elif k < 0.6 and t.startswith("{") and t.endswith("}"):
             t = t[1:-1]
-        t = rng.choice(["", "", " ", "\n", " ", "\t"]) + t + rng.choice(["", "", " ", "\r\n", "　"])
+        t = rng.choice(["", "", " ", "\n", " ", "\t"]) + t + rng.choice(["", "", " ", "\r\n", "　"])
         if _DELTA.search(t) or any(0xD800 <= ord(c) <= 0xDFFF for c in t) or t.count("[") + t.count("{") > 60:
             continue
-        r = gen_golden.run(ref.tool_post_invoke(ToolPostInvokePayload(name="t", result=t), ctx))
-        cases.append({"result": t, "continue_processing": r.continue_processing, "out_result": r.modified_payload.result if r.modified_payload is not None else None,
-                      "modified": r.modified_payload is not None, "metadata": r.metadata or {}})
-    try:
-        for i in range(0, len(cases), 500):
-            tj.check_dropin(cases[i:i + 500], JSONRepairPlugin)
-    except AssertionError as exc:
-        print("BAD", str(exc)[:1500])
+        out.append(t)
+    return out
+
+
+def outcome(r):
+    return {"continue_processing": r.continue_processing, "out_result": r.modified_payload.result if r.modified_payload is not None else None,
+            "modified": r.modified_payload is not None, "metadata": r.metadata or {}}
+
+
+def record(argv):
+    seed = int(argv[0]) if len(argv) > 0 else 1
+    n = int(argv[1]) if len(argv) > 1 else 3000
+    gen_golden.install_shims()
+    from cpex.framework import GlobalContext, PluginConfig, PluginContext, ToolPostInvokePayload
+    from plugins.json_repair.json_repair import JSONRepairPlugin as RefPlugin
+
+    ref = RefPlugin(PluginConfig(name="jr", kind="x", hooks=["tool_post_invoke"]))
+    ctx = PluginContext(global_context=GlobalContext(request_id="fuzz"))
+    ts = texts(seed, n)
+    outputs = [gen_golden.digest(outcome(gen_golden.run(ref.tool_post_invoke(ToolPostInvokePayload(name="t", result=t), ctx)))) for t in ts]
+    return {"seed": seed, "cases": n, "inputs": gen_golden.digest(ts), "outputs": outputs}
+
+
+def compare(rec) -> int:
+    import asyncio
+
+    import pytest
+
+    import hostsim_batcher
+    from mcp_context_forge_b200 import framework as fw
+    from mcp_context_forge_b200.plugins.json_repair import JSONRepairPlugin
+
+    ts = texts(rec["seed"], rec["cases"])
+    if gen_golden.digest(ts) != rec["inputs"]:
+        print("the generator no longer yields the recorded texts: record the reference again (--record) bad=1")
         return 1
-    print(f"seed={seed} cases={len(cases)} repaired={sum(c['modified'] for c in cases)} bad=0 time={time.time() - t0:.1f}s")
-    return 0
+    hostsim_batcher.install(pytest.MonkeyPatch())
+    t0 = time.time()
+    plug = JSONRepairPlugin(fw.PluginConfig(name="jr", kind="x", hooks=["tool_post_invoke"]))
+    ctx = fw.PluginContext(global_context=fw.GlobalContext(request_id="fuzz"))
+    bad = repaired = 0
+    for i in range(0, len(ts), 500):                            # all calls of a chunk concurrent: they share launches
+        async def go():
+            return await asyncio.gather(*[plug.tool_post_invoke(fw.ToolPostInvokePayload(name="t", result=t), ctx) for t in ts[i:i + 500]])
+
+        for t, r, d in zip(ts[i:i + 500], gen_golden.run(go()), rec["outputs"][i:i + 500]):
+            got = outcome(r)
+            repaired += got["modified"]
+            if gen_golden.digest(got) != d or (got["modified"] and r.modified_payload.name != "t"):
+                bad += 1
+                if bad <= 8:
+                    print("BAD", repr(t)[:300], "\n   drop-in", repr(got)[:300])
+    print(f"seed={rec['seed']} cases={len(ts)} repaired={repaired} bad={bad} time={time.time() - t0:.1f}s")
+    return 1 if bad else 0
+
+
+def main() -> int:
+    return gen_golden.fuzz_main("fuzz_json_repair_vs_reference", sys.argv[1:], record, compare)
 
 
 if __name__ == "__main__":

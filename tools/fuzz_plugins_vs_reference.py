@@ -3,7 +3,7 @@ order, payload rebuilding — on the engine's CPU simulator) against the REFEREN
 regex_filter, deny_filter, harmful_content_detector, sql_sanitizer, code_safety_linter, toon_encoder.  Random configurations (from pools that
 include rules matching "", group-reference templates, invalid patterns, IGNORECASE Unicode traps) and random payload shapes (nested dicts /
 lists / non-strings, every hook each plugin implements).  A configuration the engine rejects loudly (UnsupportedPattern) is skipped and counted.
-usage: python tools/fuzz_plugins_vs_reference.py [seed] [rounds]"""
+usage: python tools/fuzz_plugins_vs_reference.py [--record OUT] [seed] [rounds]  |  --replay tests/golden/fuzz_plugins.json.gz"""
 import asyncio
 import json
 import os
@@ -66,37 +66,25 @@ def norm(r):
                                   "metadata": md}, default=str, sort_keys=True))
 
 
-def main() -> int:
-    if not os.path.isdir(gen_golden.REF):
-        print("fuzz_plugins_vs_reference: /root/reference is not here (container-only tool)")
-        return 0
-    seed = int(sys.argv[1]) if len(sys.argv) > 1 else 1
-    rounds = int(sys.argv[2]) if len(sys.argv) > 2 else 40
-    gen_golden.install_shims()
-    import pytest
-    from cpex.framework import GlobalContext, PluginConfig, PluginContext, PromptPosthookPayload, PromptPrehookPayload, ToolPostInvokePayload, ToolPreInvokePayload
-    from plugins.code_safety_linter.code_safety_linter import CodeSafetyLinterPlugin as RCode
-    from plugins.deny_filter.deny import DenyListPlugin as RDeny
-    from plugins.harmful_content_detector.harmful_content_detector import HarmfulContentDetectorPlugin as RHarm
-    from plugins.regex_filter.search_replace import SearchReplacePlugin as RRegex
-    from plugins.sql_sanitizer.sql_sanitizer import SQLSanitizerPlugin as RSql
-    from plugins.toon_encoder.toon_encoder import ToonEncoderPlugin as RToon
+# plugin -> (the reference's class, this repository's drop-in)
+CLASSES = {"regex_filter": ("plugins.regex_filter.search_replace.SearchReplacePlugin", "regex_filter.SearchReplacePlugin"),
+           "deny_filter": ("plugins.deny_filter.deny.DenyListPlugin", "deny_filter.DenyListPlugin"),
+           "harmful": ("plugins.harmful_content_detector.harmful_content_detector.HarmfulContentDetectorPlugin", "harmful_content_detector.HarmfulContentDetectorPlugin"),
+           "sql_sanitizer": ("plugins.sql_sanitizer.sql_sanitizer.SQLSanitizerPlugin", "sql_sanitizer.SQLSanitizerPlugin"),
+           "code_safety": ("plugins.code_safety_linter.code_safety_linter.CodeSafetyLinterPlugin", "code_safety_linter.CodeSafetyLinterPlugin"),
+           "toon_encoder": ("plugins.toon_encoder.toon_encoder.ToonEncoderPlugin", "toon_encoder.ToonEncoderPlugin")}
 
-    import hostsim_batcher
-    from mcp_context_forge_b200.plugins.code_safety_linter import CodeSafetyLinterPlugin
-    from mcp_context_forge_b200.plugins.deny_filter import DenyListPlugin
-    from mcp_context_forge_b200.plugins.harmful_content_detector import HarmfulContentDetectorPlugin
-    from mcp_context_forge_b200.plugins.regex_filter import SearchReplacePlugin
-    from mcp_context_forge_b200.plugins.sql_sanitizer import SQLSanitizerPlugin
-    from mcp_context_forge_b200.plugins.toon_encoder import ToonEncoderPlugin
-    from mcp_context_forge_b200.regex_frontend import UnsupportedPattern
 
-    hostsim_batcher.install(pytest.MonkeyPatch())
-    ctx = PluginContext(global_context=GlobalContext(request_id="fuzz"))
+def load_class(path):
+    import importlib
+
+    mod, _, cls = path.rpartition(".")
+    return getattr(importlib.import_module(mod), cls)
+
+
+def plans(seed: int, rounds: int):
+    """The seeded inputs: per round and plugin (name, config, hooks, [(hook, args / result / rendered prompt)])."""
     rng = random.Random(seed)
-    loop = asyncio.new_event_loop()
-    t0 = time.time()
-    n = bad = rejected = raised = 0
 
     def payloads(kind):
         out = []
@@ -109,61 +97,112 @@ def main() -> int:
                 out.append(text(rng) if r < 0.3 else value(rng, 3) if r < 0.7 else {"content": [{"type": "text", "text": json.dumps(value(rng, 3), ensure_ascii=False)}, {"type": "image", "data": "A"}], "isError": False})
         return out
 
+    out = []
     for rd in range(rounds):
         plan = [
-            ("regex_filter", RRegex, SearchReplacePlugin, {"words": [{"search": s, "replace": r} for s, r in rng.sample(RULES, rng.randint(0, 4))]}, ["prompt_pre_fetch", "tool_pre_invoke", "tool_post_invoke", "prompt_post_fetch"]),
-            ("deny_filter", RDeny, DenyListPlugin, {"words": rng.sample(DENY, rng.randint(0, 4))}, ["prompt_pre_fetch"]),
-            ("harmful", RHarm, HarmfulContentDetectorPlugin, rng.choice(HARM_CFG), ["prompt_pre_fetch", "tool_post_invoke"]),
-            ("sql_sanitizer", RSql, SQLSanitizerPlugin, rng.choice(SQL_CFG), ["prompt_pre_fetch", "tool_pre_invoke"]),
-            ("code_safety", RCode, CodeSafetyLinterPlugin, rng.choice(CODE_CFG), ["tool_post_invoke"]),
-            ("toon_encoder", RToon, ToonEncoderPlugin, rng.choice(TOON_CFG), ["tool_post_invoke"]),
+            ("regex_filter", {"words": [{"search": s, "replace": r} for s, r in rng.sample(RULES, rng.randint(0, 4))]}, ["prompt_pre_fetch", "tool_pre_invoke", "tool_post_invoke", "prompt_post_fetch"]),
+            ("deny_filter", {"words": rng.sample(DENY, rng.randint(0, 4))}, ["prompt_pre_fetch"]),
+            ("harmful", rng.choice(HARM_CFG), ["prompt_pre_fetch", "tool_post_invoke"]),
+            ("sql_sanitizer", rng.choice(SQL_CFG), ["prompt_pre_fetch", "tool_pre_invoke"]),
+            ("code_safety", rng.choice(CODE_CFG), ["tool_post_invoke"]),
+            ("toon_encoder", rng.choice(TOON_CFG), ["tool_post_invoke"]),
         ]
-        for name, rcls, ocls, cfg, hooks in plan:
-            pc = PluginConfig(name=name, kind="x", hooks=hooks, config=cfg)
-            ref = rcls(pc)
-            try:
-                ours = ocls(pc)
-            except UnsupportedPattern:
-                rejected += 1
-                continue
+        for name, cfg, hooks in plan:
+            calls = []
             for hook in hooks:
                 for p in payloads("args" if hook in ("prompt_pre_fetch", "tool_pre_invoke") else "result"):
                     if hook == "prompt_post_fetch":                                       # a rendered prompt: messages with text content
-                        msgs = {"messages": [{"role": rng.choice(["user", "assistant"]), "content": {"type": "text", "text": text(rng)}} for _ in range(rng.randint(0, 4))]}
-                        mk = lambda: PromptPosthookPayload(prompt_id="p", result=json.loads(json.dumps(msgs)))   # noqa: E731
-                    elif hook == "prompt_pre_fetch":
-                        mk = lambda: PromptPrehookPayload(prompt_id="p", args=p)          # noqa: E731
-                    elif hook == "tool_pre_invoke":
-                        mk = lambda: ToolPreInvokePayload(name="t", args=p)              # noqa: E731
-                    else:
-                        mk = lambda: ToolPostInvokePayload(name="t", result=p)           # noqa: E731
-                    try:
-                        pa, pb = mk(), mk()
-                    except Exception:  # noqa: BLE001 - a payload shape the model rejects
-                        continue
-                    try:
-                        exp = norm(loop.run_until_complete(getattr(ref, hook)(pa, ctx)))
-                    except Exception as exc:  # noqa: BLE001 - the reference raises: so must the drop-in
-                        exp = {"raises": type(exc).__name__, "message": str(exc)}
-                    try:
-                        got = norm(loop.run_until_complete(getattr(ours, hook)(pb, ctx)))
-                    except Exception as exc:  # noqa: BLE001
-                        got = {"raises": type(exc).__name__, "message": str(exc)}
-                    n += 1
-                    raised += "raises" in exp
-                    if exp != got:
-                        bad += 1
-                        if bad <= 6:
-                            print("BAD", name, hook, repr(cfg)[:300], "\n  payload  ", repr(p)[:400], "\n  reference", json.dumps(exp, ensure_ascii=False)[:500],
-                                  "\n  drop-in  ", json.dumps(got, ensure_ascii=False)[:500])
-            if callable(getattr(ref, "get_stats", None)) and callable(getattr(ours, "get_stats", None)):      # toon_encoder's counters after the same calls
-                n += 1
-                if ref.get_stats() != ours.get_stats():
-                    bad += 1
-                    if bad <= 6:
-                        print("BAD stats", name, repr(cfg), ref.get_stats(), ours.get_stats())
-    print(f"seed={seed} rounds={rounds} hook_calls={n} configs_rejected_loudly={rejected} reference_raised={raised} bad={bad} time={time.time() - t0:.1f}s")
-    return 1 if bad else 0
+                        p = {"messages": [{"role": rng.choice(["user", "assistant"]), "content": {"type": "text", "text": text(rng)}} for _ in range(rng.randint(0, 4))]}
+                    calls.append((hook, p))
+            out.append((name, cfg, hooks, calls))
+    return out
+
+
+def make_payload(fw, hook, p):
+    if hook == "prompt_post_fetch":
+        return fw.PromptPosthookPayload(prompt_id="p", result=json.loads(json.dumps(p)))
+    if hook == "prompt_pre_fetch":
+        return fw.PromptPrehookPayload(prompt_id="p", args=p)
+    if hook == "tool_pre_invoke":
+        return fw.ToolPreInvokePayload(name="t", args=p)
+    return fw.ToolPostInvokePayload(name="t", result=p)
+
+
+def outcomes(fw, plug, calls, loop):
+    """Per call the normalised result or the raised error (None: the payload model rejects the input), then the plugin's counters."""
+    ctx = fw.PluginContext(global_context=fw.GlobalContext(request_id="fuzz"))
+    out = []
+    for hook, p in calls:
+        try:
+            pl = make_payload(fw, hook, p)
+        except Exception:  # noqa: BLE001 - a payload shape the model rejects
+            out.append(None)
+            continue
+        try:
+            out.append(norm(loop.run_until_complete(getattr(plug, hook)(pl, ctx))))
+        except Exception as exc:  # noqa: BLE001 - the reference raises: so must the drop-in
+            out.append({"raises": type(exc).__name__, "message": str(exc)})
+    return out, (plug.get_stats() if callable(getattr(plug, "get_stats", None)) else None)
+
+
+def record(argv):
+    seed = int(argv[0]) if len(argv) > 0 else 1
+    rounds = int(argv[1]) if len(argv) > 1 else 40
+    gen_golden.install_shims()
+    import cpex.framework as fw
+
+    loop = asyncio.new_event_loop()
+    ps = plans(seed, rounds)
+    outputs = []
+    for name, cfg, hooks, calls in ps:
+        res, stats = outcomes(fw, load_class(CLASSES[name][0])(fw.PluginConfig(name=name, kind="x", hooks=hooks, config=cfg)), calls, loop)
+        outputs.append([[None if r is None else gen_golden.digest(r) for r in res], None if stats is None else gen_golden.digest(stats)])
+    return {"seed": seed, "rounds": rounds, "inputs": gen_golden.digest(ps), "outputs": outputs}
+
+
+def compare(rec) -> int:
+    import pytest
+
+    import hostsim_batcher
+    from mcp_context_forge_b200 import framework as fw
+    from mcp_context_forge_b200.regex_frontend import UnsupportedPattern
+
+    ps = plans(rec["seed"], rec["rounds"])
+    if gen_golden.digest(ps) != rec["inputs"]:
+        print("the generator no longer yields the recorded inputs: record the reference again (--record) bad=1")
+        return 1
+    hostsim_batcher.install(pytest.MonkeyPatch())
+    loop = asyncio.new_event_loop()
+    t0 = time.time()
+    n = bad = rejected = raised = 0
+    for (name, cfg, hooks, calls), (exp, exp_stats) in zip(ps, rec["outputs"]):
+        try:
+            ours = load_class("mcp_context_forge_b200.plugins." + CLASSES[name][1])(fw.PluginConfig(name=name, kind="x", hooks=hooks, config=cfg))
+        except UnsupportedPattern:
+            rejected += 1
+            continue
+        got, stats = outcomes(fw, ours, calls, loop)
+        for (hook, p), e, g in zip(calls, exp, got):
+            if e is None and g is None:
+                continue
+            n += 1
+            raised += isinstance(g, dict) and "raises" in g
+            if g is None or gen_golden.digest(g) != e:
+                bad += 1
+                if bad <= 6:
+                    print("BAD", name, hook, repr(cfg)[:300], "\n  payload  ", repr(p)[:400], "\n  drop-in  ", json.dumps(g, ensure_ascii=False)[:500])
+        if exp_stats is not None:                              # toon_encoder's counters after the same calls
+            n += 1
+            if stats is None or gen_golden.digest(stats) != exp_stats:
+                bad += 1
+                if bad <= 6:
+                    print("BAD stats", name, repr(cfg), stats)
+    print(f"seed={rec['seed']} rounds={rec['rounds']} hook_calls={n} configs_rejected_loudly={rejected} drop_in_raised={raised} bad={bad} time={time.time() - t0:.1f}s")
+    return 1 if bad or not n else 0
+
+
+def main() -> int:
+    return gen_golden.fuzz_main("fuzz_plugins_vs_reference", sys.argv[1:], record, compare)
 
 
 if __name__ == "__main__":

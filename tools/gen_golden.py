@@ -17,6 +17,8 @@ from __future__ import annotations
 
 import ast
 import asyncio
+import gzip
+import hashlib
 import json
 import logging
 import os
@@ -82,6 +84,44 @@ def dump(name, obj):
         json.dump(obj, f, ensure_ascii=True, indent=0, separators=(",", ":"))
         f.write("\n")
     print(f"wrote {path}: {os.path.getsize(path)} bytes")
+
+
+def digest(obj) -> str:
+    """32-bit digest of a value's canonical JSON (dict order ignored, as `==` does).  A fuzzer's recording keeps the reference's output
+    for each case as this digest, and its inputs as the digest of the whole seeded sequence, which the fuzzer regenerates."""
+    data = json.dumps(obj, ensure_ascii=True, sort_keys=True, separators=(",", ":"), default=repr).encode()
+    return hashlib.sha256(data).hexdigest()[:8]
+
+
+def save_recording(path, obj):
+    """A differential fuzzer's recorded run as gzip-compressed JSON, byte-reproducible."""
+    data = json.dumps(obj, ensure_ascii=True, separators=(",", ":")).encode()
+    with open(path, "wb") as f:
+        f.write(gzip.compress(data, compresslevel=9, mtime=0))
+    print(f"wrote {path}: {os.path.getsize(path)} bytes")
+
+
+def load_recording(path):
+    with open(path, "rb") as f:
+        return json.loads(gzip.decompress(f.read()))
+
+
+def fuzz_main(name, argv, record, compare):
+    """Command line of the differential fuzzers.  `[args]`: run the reference live and compare; `--record OUT [args]`: write the
+    reference's side of the run to OUT; `--replay IN`: compare this repository against a recording (the reference is not needed)."""
+    if argv[:1] == ["--replay"]:
+        return compare(load_recording(argv[1]))
+    out = None
+    if argv[:1] == ["--record"]:
+        out, argv = argv[1], argv[2:]
+    if not os.path.isdir(REF):
+        print(f"{name}: the reference checkout ({REF}) is not here; compare against a recording with --replay")
+        return 0 if out is None else 1
+    rec = record(argv)
+    if out is not None:
+        save_recording(out, rec)
+        return 0
+    return compare(rec)
 
 
 # ------------------------------------------------------------------------------------------------
